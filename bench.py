@@ -19,6 +19,9 @@ from pinned HOST memory (H2D of every image batch and D2H of the result inside t
 `precision_modes` repeats the device-resident measurement in the `parity` (split-bf16, fp32-level) network mode -- the
 mode whose scores stay within the 1e-4 tolerance of BASELINE.json; the headline runs the networks in bf16 (`fast`).
 `cpu_baseline` / `--impl reference` time the CPU restatement of the reference path (oracle/) on a bounded sample.
+`--dump-outputs DIR` writes what the last timed step returned -- top-k values and indices plus the query and gallery
+descriptors, or the FID value for c4 -- as DIR/<name>.npy; the inputs are seeded, so the dumps of two builds of the
+project compare output for output.
 """
 from __future__ import annotations
 
@@ -40,6 +43,7 @@ K_TOP = 10
 IMG = 256
 FID_IMG = 299
 METRIC = "embed+top-k query images/sec"
+DUMP_LIMIT = 60_000_000      # bytes of array data in one --dump-outputs directory (npy headers add 128 bytes a file)
 
 
 def load_peaks():
@@ -300,7 +304,13 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--cpu-embed-sample", type=int, default=128)
     ap.add_argument("--cpu-sim-sample", type=int, default=1000)
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm times samples, not the workload)")
     if args.net is None:
         args.net = "dino" if args.config == "c3" else "sscd"
     if args.scaling is None:
@@ -422,6 +432,30 @@ def check_result(values, indices, qf_all_fn, gf, g_base, world, dev, n_check: in
             "against": "per-rank fp64 torch matmul + stable sort on a query subsample, merged on the host"}
 
 
+def dump_outputs(out_dir: str, arrays: dict, limit: int = DUMP_LIMIT) -> dict:
+    """Writes every tensor of `arrays` (rows first) as out_dir/<name>.npy: float64 stays float64, other floating types
+    become float32, integers become float64 (exact below 2**53).  The arrays share `limit` bytes: the smallest ones are
+    written whole, and an array larger than an equal share of what is left keeps evenly spaced rows (row r*n//m of n,
+    r < m).  The same shapes give the same rows, so the dumps of two builds compare file by file.
+    Returns {name: [rows written, rows in the output]}."""
+    os.makedirs(out_dir, exist_ok=True)
+    written = {}
+    left = limit
+    order = sorted(arrays, key=lambda name: arrays[name].numel())
+    for i, name in enumerate(order):
+        t = arrays[name].detach()
+        t = t.to(torch.float64 if t.dtype == torch.float64 or not t.is_floating_point() else torch.float32)
+        n = t.shape[0]
+        row_bytes = max(1, t[:1].numel()) * t.element_size()
+        m = min(n, (left // (len(order) - i)) // row_bytes)
+        if m < n:
+            t = t[(torch.arange(m, dtype=torch.int64) * n // m).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+        left -= m * row_bytes
+        written[name] = [m, n]
+    return written
+
+
 def run_retrieval_bench(args, rank, local_rank, world):
     import torch.distributed as dist
     from dcr_b200 import dist as ddist
@@ -484,7 +518,11 @@ def run_retrieval_bench(args, rank, local_rank, world):
     if rank == 0:
         sampler.start()
     l0 = similarity.kernel_launch_count()
-    ms_total, kernel_ms = timed(lambda: step(gal_u8, qry_u8), args.steps)
+
+    def timed_step():
+        keep["out"] = step(gal_u8, qry_u8)
+
+    ms_total, kernel_ms = timed(timed_step, args.steps)
     launches = similarity.kernel_launch_count() - l0
     ms_per_step = ms_total / args.steps
     value = q_total / (ms_per_step / 1e3)
@@ -492,6 +530,12 @@ def run_retrieval_bench(args, rank, local_rank, world):
     if rank == 0:
         sampler.stop_flag.set()
         sampler.join(timeout=2)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # every rank holds the merged top-k of all queries; the descriptors are this rank's queries and gallery shard
+        dumped = dump_outputs(args.dump_outputs, {"values": keep["out"][0], "indices": keep["out"][1],
+                                                  "query_features": keep["qf"], "gallery_features": keep["gf"]})
+    del keep["out"]
 
     # ---- the step validates its own output (all ranks take part: collectives inside) -------------------------------
     out_v, out_i = step(gal_u8, qry_u8)
@@ -589,6 +633,8 @@ def run_retrieval_bench(args, rank, local_rank, world):
                               "unit": "TFLOP/s", "frac": embed_tflops / world / peaks["sustained"]}
     if e2e is not None:
         line["e2e"] = e2e
+    if dumped is not None:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "rows_written_of": dumped}
     if others:
         line["precision_modes"] = {args.precision: {"value": value, "unit": "query images/s", "ms_per_step": ms_per_step,
                                                     "note": notes.get(args.precision, "")}}
@@ -657,6 +703,9 @@ def run_fid_bench(args, rank, local_rank, world):
     l0 = similarity.kernel_launch_count()
     ms = timed(lambda: step(real, gen), args.steps) / args.steps
     launches = similarity.kernel_launch_count() - l0
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = dump_outputs(args.dump_outputs, {"fid": torch.tensor([result["fid"]], dtype=torch.float64)})
     n_total = (n_gen + n_real) * world
     e2e = None
     if not args.no_e2e:
@@ -689,6 +738,8 @@ def run_fid_bench(args, rank, local_rank, world):
                          "frac": tfl / world / peaks["sustained"], "traffic": None}}
     if e2e is not None:
         line["e2e"] = e2e
+    if dumped is not None:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "rows_written_of": dumped}
     if world == 1:
         v, det = cpu_reference_fid_sample(max(16, args.cpu_embed_sample // 4), n_total)
         line["cpu_baseline"] = {"value": v, "unit": "images/s", "cores": det["cores"], "kind": "port", "sample": det["sample"]}
