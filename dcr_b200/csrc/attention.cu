@@ -5,14 +5,14 @@
 // Input  qkv : bf16 planes [B*T, 3*heads*dh] (columns [q | k | v], each heads x dh) -- the fused qkv GEMM output.
 // Output out : bf16 planes [B*T, heads*dh].
 //
-// attention_tc_kernel (fast mode, one bf16 plane): one CTA per (image, head), everything on tcgen05:
-//   S = Q K^T   UMMA 128 x 256 x 16 (two M tiles cover T <= 256 tokens), fp32 in TMEM
+// attention_tc1_kernel (fast mode, one bf16 plane, T <= 256): one CTA per (image, head, 128-row query tile), on tcgen05:
+//   S = Q K^T   UMMA 128 x 256 x 16, fp32 in TMEM
 //   softmax     4 warps, thread = query row: two passes over the TMEM row (max, then exp2/sum), P written as bf16
 //               into a 128B-swizzled K-major shared-memory tile; keys >= T are masked to 0
 //   O = P V     UMMA 128 x 64 x 16 with V consumed in place as an MN-major operand (no transpose)
 //   epilogue    O / rowsum -> bf16 -> global
-// attention_fp32_kernel: exact-fp32 path (used by parity mode, and by fast mode until the tcgen05 kernel below
-// is enabled): K and V of one (image, head) live in shared memory as fp32, one warp per query row.
+// attention_fp32_kernel: exact-fp32 path (parity mode, several planes): K and V of one (image, head) live in shared
+// memory as fp32, one warp per query row.  attention_stream_kernel: the same for T > 256.
 #include <cuda_bf16.h>
 
 #include "dcr_internal.cuh"
@@ -204,11 +204,8 @@ __global__ void __launch_bounds__(256) attention_stream_kernel(const AttnParams 
   }
 }
 
-
 // ---------------------------------------------------------------------------------------------------------------
 // tcgen05 attention
-constexpr int kAttnThreads = 288;   // warps 0-3 / 4-7: softmax + epilogue of query tile 0 / 1, warp 8: TMA + MMA issue
-
 DCR_DEVICE uint64_t umma_desc_sw128_mn(uint32_t smem_addr) {
   // MN-major operand, 128B swizzle: 64 contiguous elements along MN per row, rows = K, 8-row groups 1024 B apart
   uint64_t d = 0;
@@ -227,194 +224,13 @@ struct AttnTcParams {
   int causal;           // 1: keys beyond the query's own position are masked
 };
 
-__global__ void __launch_bounds__(kAttnThreads, 1)
-    attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const AttnTcParams p) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* s_q = smem;                 // 2 x [128 x 64] bf16
-  uint8_t* s_k = s_q + 2 * 16384;      // [256 x 64]
-  uint8_t* s_v = s_k + 32768;          // [256 x 64]
-  uint8_t* s_p = s_v + 32768;          // per query tile: 4 k-blocks x [128 x 64]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(s_p + 2 * 65536);
-  uint64_t* bar_load = bars;           // TMA landed
-  uint64_t* s_full = bars + 1;         // [2] S tile ready in TMEM
-  uint64_t* p_ready = bars + 3;        // [2] P written + S consumed (128 arrivals)
-  uint64_t* o_full = bars + 5;         // [2] O tile ready in TMEM
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 7);
-
-  const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int b = blockIdx.x / p.heads, h = blockIdx.x % p.heads;
-  const int row0 = b * p.T;
-  const int n_mtiles = (p.T + 127) / 128;
-
-  if (warp == 8 && lane == 0) {
-    tma_prefetch_desc(&tmap_qkv);
-    mbar_init(bar_load, 1);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&s_full[i], 1);
-      mbar_init(&p_ready[i], 128);
-      mbar_init(&o_full[i], 1);
-    }
-    fence_mbar_init();
-  }
-  if (warp == 0) {
-    tmem_alloc<1>(tmem_slot, 512);
-    tmem_relinquish<1>();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 8) {
-    {   // control warp: all lanes walk the (warp-uniform) code, one elected lane issues (see conv_gemm.cu)
-      const int cq = h * 64, ck = p.heads * 64 + h * 64, cv = 2 * p.heads * 64 + h * 64;
-      if (elect_one()) {
-        mbar_arrive_expect_tx(bar_load, 6 * 16384);
-        tma_load_2d<1>(s_q, &tmap_qkv, bar_load, cq, row0, kEvictFirst);
-        tma_load_2d<1>(s_q + 16384, &tmap_qkv, bar_load, cq, row0 + 128, kEvictFirst);
-        tma_load_2d<1>(s_k, &tmap_qkv, bar_load, ck, row0, kEvictFirst);
-        tma_load_2d<1>(s_k + 16384, &tmap_qkv, bar_load, ck, row0 + 128, kEvictFirst);
-        tma_load_2d<1>(s_v, &tmap_qkv, bar_load, cv, row0, kEvictFirst);
-        tma_load_2d<1>(s_v + 16384, &tmap_qkv, bar_load, cv, row0 + 128, kEvictFirst);
-      }
-      __syncwarp();
-      mbar_wait(bar_load, 0);
-      tc_fence_after();
-      constexpr uint32_t idesc_s = umma_idesc_bf16(128, 256);
-      constexpr uint32_t idesc_o = umma_idesc_bf16(128, 64) | (1u << 16);   // B operand MN-major
-      for (int mt = 0; mt < n_mtiles; ++mt) {
-        const uint64_t da = umma_desc_sw128(smem_u32(s_q + mt * 16384));
-        const uint64_t db = umma_desc_sw128(smem_u32(s_k));
-        if (elect_one()) {
-#pragma unroll
-          for (int k = 0; k < 4; ++k) umma_f16<1>(tmem_base + mt * 256, da + 2 * k, db + 2 * k, idesc_s, k != 0);
-          umma_commit<1>(&s_full[mt]);
-        }
-        __syncwarp();
-      }
-      for (int mt = 0; mt < n_mtiles; ++mt) {
-        mbar_wait(&p_ready[mt], 0);
-        tc_fence_after();
-        if (elect_one()) {
-#pragma unroll
-          for (int kb = 0; kb < 4; ++kb) {
-            const uint64_t da = umma_desc_sw128(smem_u32(s_p + mt * 65536 + kb * 16384));
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              // A: +32 B per 16 keys inside the 64-key block; B (V, MN-major): +16 rows * 128 B per 16 keys
-              const uint64_t dv = umma_desc_sw128_mn(smem_u32(s_v + (kb * 64 + k * 16) * 128));
-              umma_f16<1>(tmem_base + mt * 256, da + 2 * k, dv, idesc_o, (kb | k) != 0);
-            }
-          }
-          umma_commit<1>(&o_full[mt]);
-        }
-        __syncwarp();
-      }
-    }
-  } else {
-    const int mt = static_cast<int>(warp >> 2);          // the query tile this warp group owns
-    const uint32_t quad = warp & 3;
-    const uint32_t row = quad * 32 + lane;
-    const uint32_t tmem_row = tmem_base + ((quad * 32u) << 16);
-    const uint32_t sw = row & 7;
-    if (mt < n_mtiles) {
-      mbar_wait(&s_full[mt], 0);
-      tc_fence_after();
-      const uint32_t taddr = tmem_row + mt * 256;
-      const int lim = p.causal ? min(p.T, mt * 128 + static_cast<int>(row) + 1) : p.T;   // keys this query row may see
-      // pass 1: row maximum over the valid keys
-      float mx = -INFINITY;
-#pragma unroll 1
-      for (int ch = 0; ch < 8; ++ch) {
-        if (ch * 32 >= p.T) break;
-        uint32_t r[32];
-        tmem_ld_32x32(taddr + ch * 32, r);
-        tmem_ld_wait_regs(r);
-#pragma unroll
-        for (int c = 0; c < 32; ++c)
-          if (ch * 32 + c < lim) mx = fmaxf(mx, __uint_as_float(r[c]));
-      }
-      const float mxs = mx * p.scale_log2e;
-      // pass 2: exp, row sum, P -> shared memory (bf16, K-major, 128B swizzle)
-      float sum = 0.f;
-#pragma unroll 1
-      for (int ch = 0; ch < 8; ++ch) {
-        uint32_t r[32];
-        float pv[32];
-        if (ch * 32 < p.T) {
-          tmem_ld_32x32(taddr + ch * 32, r);
-          tmem_ld_wait_regs(r);
-#pragma unroll
-          for (int c = 0; c < 32; ++c) {
-            const float e = (ch * 32 + c < lim) ? exp2f(fmaf(__uint_as_float(r[c]), p.scale_log2e, -mxs)) : 0.f;
-            // the sum must be of the ROUNDED weights that the tensor core will use
-            const float eb = __bfloat162float(__float2bfloat16_rn(e));
-            pv[c] = eb;
-            sum += eb;
-          }
-        } else {
-#pragma unroll
-          for (int c = 0; c < 32; ++c) pv[c] = 0.f;
-        }
-        uint8_t* prow = s_p + mt * 65536 + (ch >> 1) * 16384 + row * 128;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          uint4 v;
-          __nv_bfloat162 t0 = __floats2bfloat162_rn(pv[j * 8 + 0], pv[j * 8 + 1]);
-          __nv_bfloat162 t1 = __floats2bfloat162_rn(pv[j * 8 + 2], pv[j * 8 + 3]);
-          __nv_bfloat162 t2 = __floats2bfloat162_rn(pv[j * 8 + 4], pv[j * 8 + 5]);
-          __nv_bfloat162 t3 = __floats2bfloat162_rn(pv[j * 8 + 6], pv[j * 8 + 7]);
-          v.x = *reinterpret_cast<uint32_t*>(&t0);
-          v.y = *reinterpret_cast<uint32_t*>(&t1);
-          v.z = *reinterpret_cast<uint32_t*>(&t2);
-          v.w = *reinterpret_cast<uint32_t*>(&t3);
-          *reinterpret_cast<uint4*>(prow + ((((ch & 1) * 4 + j) ^ sw) << 4)) = v;
-        }
-      }
-      fence_proxy_async();     // P (generic proxy) -> visible to the tensor core's async proxy
-      tc_fence_before();
-      mbar_arrive(&p_ready[mt]);
-      // epilogue of this tile
-      mbar_wait(&o_full[mt], 0);
-      tc_fence_after();
-      const int t = mt * 128 + static_cast<int>(row);
-      const float inv = 1.f / sum;
-#pragma unroll 1
-      for (int ch = 0; ch < 2; ++ch) {
-        uint32_t r[32];
-        tmem_ld_32x32(taddr + ch * 32, r);
-        tmem_ld_wait_regs(r);
-        if (t < p.T) {
-          __nv_bfloat16* op = p.out + static_cast<size_t>(row0 + t) * (p.heads * 64) + h * 64 + ch * 32;
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            uint4 v;
-            __nv_bfloat162 t0 = __floats2bfloat162_rn(__uint_as_float(r[j * 8 + 0]) * inv, __uint_as_float(r[j * 8 + 1]) * inv);
-            __nv_bfloat162 t1 = __floats2bfloat162_rn(__uint_as_float(r[j * 8 + 2]) * inv, __uint_as_float(r[j * 8 + 3]) * inv);
-            __nv_bfloat162 t2 = __floats2bfloat162_rn(__uint_as_float(r[j * 8 + 4]) * inv, __uint_as_float(r[j * 8 + 5]) * inv);
-            __nv_bfloat162 t3 = __floats2bfloat162_rn(__uint_as_float(r[j * 8 + 6]) * inv, __uint_as_float(r[j * 8 + 7]) * inv);
-            v.x = *reinterpret_cast<uint32_t*>(&t0);
-            v.y = *reinterpret_cast<uint32_t*>(&t1);
-            v.z = *reinterpret_cast<uint32_t*>(&t2);
-            v.w = *reinterpret_cast<uint32_t*>(&t3);
-            *reinterpret_cast<uint4*>(op + j * 8) = v;
-          }
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc<1>(tmem_base, 512);
-}
-
-// One query tile per CTA, two CTAs per SM.  The kernel above keeps Q (2 tiles), K, V and both P tiles resident (224 KB):
-// one CTA per SM, and inside a CTA load -> QK^T -> softmax -> PV -> store is a serial chain, so the SM idles through every
-// latency in turn (144 us per ViT-S/16 layer at batch 256, ~106 TFLOP/s).  Here a CTA owns ONE 128-row query tile of one
-// (image, head); its P tile (128 x 256 bf16 = 64 KB) is written over the Q and K tiles, which are dead once the S MMAs
-// have retired, so a CTA needs 96 KB and two of them share an SM (and its 512 TMEM columns, 256 each): one CTA's loads and
-// MMAs run under the other's softmax.  K / V of an (image, head) are fetched by both of its CTAs (second fetch: L2).
+// One query tile per CTA, two CTAs per SM.  A CTA owns ONE 128-row query tile of one (image, head); its P tile
+// (128 x 256 bf16 = 64 KB) is written over the Q and K tiles, which are dead once the S MMAs have retired, so a CTA needs
+// 96 KB and two of them share an SM (and its 512 TMEM columns, 256 each): one CTA's loads and MMAs run under the other's
+// softmax.  K / V of an (image, head) are fetched by both of its CTAs (second fetch: L2).  The earlier form with one CTA
+// per (image, head) kept Q (2 tiles), K, V and both P tiles resident (224 KB), so load -> QK^T -> softmax -> PV -> store
+// ran as a serial chain on one CTA per SM: 144 us per ViT-S/16 layer at batch 256, ~106 TFLOP/s (removed after commit
+// 997ac6f).
 constexpr int kAttn1Threads = 160;   // warps 0-3 softmax + epilogue, warp 4 TMA + MMA issue
 DCR_DEVICE float ex2_approx(float x) {
   float y;
@@ -631,7 +447,7 @@ int attention(const __nv_bfloat16* qkv, long long qkv_plane_stride, __nv_bfloat1
   DCR_REQUIRE(dh == 64, "attention: head dim %d not supported (64 only)", dh);
   DCR_REQUIRE(T >= 1 && T <= 16384, "attention: sequence length %d out of range", T);
   if (B == 0) return 0;
-  if (planes == 1 && T <= 256 && !tuning_flag("DCR_ATTN_FP32")) {
+  if (planes == 1 && T <= 256) {   // one query tile per CTA, two CTAs per SM
     const DeviceInfo* di = device_info();
     if (!di) return -2;
     CUtensorMap tm;
@@ -639,19 +455,10 @@ int attention(const __nv_bfloat16* qkv, long long qkv_plane_stride, __nv_bfloat1
     AttnTcParams tp;
     tp.out = out; tp.B = B; tp.T = T; tp.heads = heads; tp.causal = causal;
     tp.scale_log2e = scale * 1.4426950408889634f;
-    if (!tuning_flag("DCR_ATTN_ONE_CTA")) {   // one query tile per CTA, two CTAs per SM
-      const size_t smem1 = 1024 + 16384 + 32768 + 16384 + 32768 + 256;
-      DCR_CUDA_CHECK(cudaFuncSetAttribute(attention_tc1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          static_cast<int>(smem1)));
-      attention_tc1_kernel<<<B * heads * ((T + 127) / 128), kAttn1Threads, smem1, stream>>>(tm, tp);
-      count_launch();
-      DCR_CUDA_CHECK(cudaGetLastError());
-      return 0;
-    }
-    const size_t smem = 1024 + 2 * 16384 + 32768 + 32768 + 2 * 65536 + 256;
-    DCR_CUDA_CHECK(cudaFuncSetAttribute(attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        static_cast<int>(smem)));
-    attention_tc_kernel<<<B * heads, kAttnThreads, smem, stream>>>(tm, tp);
+    const size_t smem1 = 1024 + 16384 + 32768 + 16384 + 32768 + 256;
+    DCR_CUDA_CHECK(cudaFuncSetAttribute(attention_tc1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        static_cast<int>(smem1)));
+    attention_tc1_kernel<<<B * heads * ((T + 127) / 128), kAttn1Threads, smem1, stream>>>(tm, tp);
     count_launch();
     DCR_CUDA_CHECK(cudaGetLastError());
     return 0;

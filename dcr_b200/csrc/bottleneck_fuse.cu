@@ -412,7 +412,7 @@ __global__ void __launch_bounds__(kFThreads, 1) expand_reduce_kernel(const __gri
 }  // namespace
 
 bool expand_only_eligible(const ConvGemmDesc& a, size_t max_smem) {
-  if (tuning_flag("DCR_NO_BLOCK_FUSION") || tuning_flag("DCR_NO_EXPAND_ONLY")) return false;
+  if (tuning_flag("DCR_NO_BLOCK_FUSION")) return false;
   const bool plain = a.kh == 1 && a.kw == 1 && a.stride == 1 && a.pad_h == 0 && a.pad_w == 0 && a.in_stride_w == 0 && a.n_terms == 1 &&
                      a.term_a[0] == 0 && a.term_w[0] == 0 && !a.exact && a.out != nullptr && a.out_planes <= 1 && a.out_f32 == nullptr &&
                      a.out_col_off == 0 && a.act == 1;

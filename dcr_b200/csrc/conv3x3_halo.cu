@@ -2,7 +2,7 @@
 //
 // The generic kernel (conv_gemm.cu) gathers one [128 pixels x 64 channels] A tile per filter tap, i.e. every input
 // pixel travels L2 -> shared memory nine times; for the convolutions with few output channels that ingest is the
-// bound (DESIGN.md section 5: load-only timing mode = 96 % of the layer time).  Here a tile is R whole output rows of
+// bound (DESIGN.md section 5: loads alone took 96 % of the layer time).  Here a tile is R whole output rows of
 // one image and the producer loads, per 64-channel block, ONE halo block
 //       [(R + 2) input rows] x [(W + 2) pixels, the two extra ones zero-filled by the TMA unit] x [64 channels]
 // as a single 4-D tiled TMA box.  In shared memory that is a width-padded raster of 128-byte rows, so the A operand of
@@ -35,11 +35,6 @@ constexpr int kHM = 128;                    // MMA rows (padded-raster positions
 constexpr int kHK = 64;                     // channels per block = one 128-byte swizzled row
 constexpr int kSlabBytes = kHM * 128;       // one 64-channel slab of the output staging tile
 constexpr int kHThreads = 352;              // warp 0 producer, warp 1 (and 10) MMA issuers, warps 2..9 epilogue
-// Timing experiments (garbage results), compile-time only: bit 0 = no weight loads, bit 1 = no halo loads.
-#ifndef DCR_HALO_TIMING_MODE
-#define DCR_HALO_TIMING_MODE 0
-#endif
-constexpr int kHaloTimingMode = DCR_HALO_TIMING_MODE;
 
 struct HaloMaps {
   CUtensorMap a;     // input  [B][H][W][C]   box 64 x (W+2) x (R+2) x 1
@@ -125,7 +120,6 @@ __global__ void __launch_bounds__(kHThreads, 1)
     // ===================================== TMA producer =====================================
     // (whole warp walks the loop, one elected lane issues: see conv_gemm.cu)
     {
-      uint32_t ai = 0, wi = 0;
       PipeState as(p.a_bufs), ws(kRW ? 1 : p.w_stages);
       if constexpr (kRW) {   // every filter tap once
         if (elect_one()) {
@@ -138,30 +132,22 @@ __global__ void __launch_bounds__(kHThreads, 1)
       for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
         const int b = tile / p.tiles_per_img;
         const int p0 = (tile - b * p.tiles_per_img) * p.R;
-        for (int cb = 0; cb < p.cblocks; ++cb, ++ai, as.next()) {
+        for (int cb = 0; cb < p.cblocks; ++cb, as.next()) {
           const uint32_t sa = as.s, pha = as.ph;
           mbar_wait(&a_empty[sa], pha ^ 1);
           if (elect_one()) {
-            if ((kHaloTimingMode & 2) && ai >= static_cast<uint32_t>(p.a_bufs)) {
-              mbar_arrive(&a_full[sa]);    // timing experiment: reuse stale halo data, no load
-            } else {
-              mbar_arrive_expect_tx(&a_full[sa], p.halo_bytes);
-              // rows p0-1 .. p0+R, columns -1 .. W: everything outside the image arrives as zeros (the padding)
-              tma_load_4d(a_ring + sa * p.a_buf_bytes, &maps.a, &a_full[sa], cb * kHK, -1, p0 - 1, b, kEvictNormal);
-            }
+            mbar_arrive_expect_tx(&a_full[sa], p.halo_bytes);
+            // rows p0-1 .. p0+R, columns -1 .. W: everything outside the image arrives as zeros (the padding)
+            tma_load_4d(a_ring + sa * p.a_buf_bytes, &maps.a, &a_full[sa], cb * kHK, -1, p0 - 1, b, kEvictNormal);
           }
           __syncwarp();
           if constexpr (kRW) continue;
-          for (int tap = 0; tap < 9; ++tap, ++wi, ws.next()) {
+          for (int tap = 0; tap < 9; ++tap, ws.next()) {
             const uint32_t sw = ws.s, phw = ws.ph;
             mbar_wait(&w_empty[sw], phw ^ 1);
             if (elect_one()) {
-              if ((kHaloTimingMode & 1) && wi >= static_cast<uint32_t>(p.w_stages)) {
-                mbar_arrive(&w_full[sw]);  // timing experiment: stale weights, no load
-              } else {
-                mbar_arrive_expect_tx(&w_full[sw], kWStage);
-                tma_load_2d<1>(w_ring + sw * kWStage, &maps.w, &w_full[sw], (tap * p.cblocks + cb) * kHK, 0, kEvictLast);
-              }
+              mbar_arrive_expect_tx(&w_full[sw], kWStage);
+              tma_load_2d<1>(w_ring + sw * kWStage, &maps.w, &w_full[sw], (tap * p.cblocks + cb) * kHK, 0, kEvictLast);
             }
             __syncwarp();
           }
@@ -355,7 +341,7 @@ bool conv3x3_halo_eligible(const ConvGemmDesc& d) {
   const bool shape = d.kh == 3 && d.kw == 3 && d.stride == 1 && d.pad_h == 1 && d.pad_w == 1 && d.in_stride_w == 0;
   const bool fast = d.n_terms == 1 && d.term_a[0] == 0 && d.term_w[0] == 0 && !d.exact && d.out != nullptr &&
                     d.out_planes <= 1 && d.out_f32 == nullptr && d.res == nullptr && (d.act == 0 || d.act == 1);
-  const bool dims = d.C % 64 == 0 && d.ld_in == d.C && d.N % 64 == 0 && d.N <= (tuning_flag("DCR_CONV_HALO_N256") ? 256 : 128) && d.ld_out % 8 == 0 &&
+  const bool dims = d.C % 64 == 0 && d.ld_in == d.C && d.N % 64 == 0 && d.N <= 128 && d.ld_out % 8 == 0 &&
                     d.out_col_off % 8 == 0 && d.W + 2 <= 64 && d.W >= 8 && d.H >= 2 && d.B >= 1;
   return shape && fast && dims;
 }
@@ -378,16 +364,15 @@ int conv3x3_halo(const ConvGemmDesc& d, cudaStream_t stream) {
   HaloMaps maps;
   memset(&maps, 0, sizeof(maps));
   if (int rc = make_tmap_nhwc_box_bf16(&maps.a, d.in, d.B, d.H, d.W, d.C, d.C, p.Wp, p.R + 2)) return rc;
-  const int BN = d.N <= 64 ? 64 : (d.N <= 128 ? 128 : 256);
+  const int BN = d.N <= 64 ? 64 : 128;   // conv3x3_halo_eligible: N is 64 or 128
   const int ktot = 9 * p.cblocks * 64;
   if (int rc = make_tmap_2d_bf16(&maps.w, d.weight, d.N, ktot, ktot, BN, 64)) return rc;
   if (int rc = make_tmap_nhwc_box_bf16(&maps.out, d.out, d.B, d.H, d.W, d.ld_out, d.ld_out, d.W, p.R)) return rc;
   // all taps resident + two MMA issuers when the weights are small (ResNet layer1: 9 x [64 x 64] = 72 KB)
-  const bool resident = BN == 64 && static_cast<size_t>(9) * p.cblocks * BN * 128 <= 80 * 1024 && !tuning_flag("DCR_HALO_NO_RESIDENT");
+  const bool resident = BN == 64 && static_cast<size_t>(9) * p.cblocks * BN * 128 <= 80 * 1024;
   if (BN == 64) return resident ? launch_halo<64, true>(maps, p, di->num_sms, di->max_smem_optin, stream)
                                 : launch_halo<64, false>(maps, p, di->num_sms, di->max_smem_optin, stream);
-  if (BN == 128) return launch_halo<128, false>(maps, p, di->num_sms, di->max_smem_optin, stream);
-  return launch_halo<256, false>(maps, p, di->num_sms, di->max_smem_optin, stream);
+  return launch_halo<128, false>(maps, p, di->num_sms, di->max_smem_optin, stream);
 }
 
 }  // namespace dcr

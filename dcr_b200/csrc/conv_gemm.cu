@@ -36,12 +36,6 @@ constexpr int kBM = 128;
 constexpr int kBK = 64;
 constexpr int kThreads = 320;   // warp 0 TMA, warp 1 MMA, warps 2-9 epilogue
 constexpr int kAStage = kBM * kBK * 2;   // 16 KB
-// Timing experiments (results are garbage), compile-time only: 1 = loads only (no MMA, no epilogue), 2 = loads only and
-// every im2col request replaced by a tiled request of the same size (row-shifted view).
-#ifndef DCR_GEMM_TIMING_MODE
-#define DCR_GEMM_TIMING_MODE 0
-#endif
-constexpr int kGemmTimingMode = DCR_GEMM_TIMING_MODE;
 // direct epilogue: per epilogue warp a [32 rows][64 B + 16 B pad] buffer through which the bf16 planes are transposed, so that
 // one warp instruction touches 8 rows x 64 contiguous bytes of global memory instead of 32 rows x 16 bytes
 constexpr int kXposePitch = 80;
@@ -53,7 +47,6 @@ struct GemmMaps {
   CUtensorMap w[3];
   CUtensorMap out;   // TMA-store epilogue (single-plane bf16 output)
   CUtensorMap res;   // residual tile loads for that epilogue
-  CUtensorMap a_flat; // timing experiment DCR_GEMM_DEBUG=2 only: the im2col input viewed as a plain [pixels, C] matrix
 };
 
 struct GemmParams {
@@ -306,13 +299,10 @@ __global__ void __launch_bounds__(kThreads, 1)
                 if (leader) mbar_arrive_expect_tx(&full[s], kStageBytes * kCG);
                 else mbar_arrive_cluster(&full[s], 0);
                 uint8_t* sa = smem_ab + s * kStageBytes;
-                if constexpr (kIm2col) {
-                  if constexpr (kGemmTimingMode == 2)
-                    tma_load_2d<1>(sa, &maps.a_flat, &full[s], cb * kBK, max(0, m0 + (r - 1) * p.Q + sx - 1), kEvictNormal);
-                  else
-                    tma_load_im2col_4d<1>(sa, ma, &full[s], cb * kBK, w0, h0, img, static_cast<uint16_t>(sx),
-                                          static_cast<uint16_t>(r));
-                } else
+                if constexpr (kIm2col)
+                  tma_load_im2col_4d<1>(sa, ma, &full[s], cb * kBK, w0, h0, img, static_cast<uint16_t>(sx),
+                                        static_cast<uint16_t>(r));
+                else
                   tma_load_2d<kCG>(sa, ma, &full[s], cb * kBK, m0, kEvictNormal);
                 tma_load_2d<kCG>(sa + kAStage, mw, &full[s], (tap * cblocks + cb) * kBK, n0 + static_cast<int>(cta_rank) * kBRows,
                                  kEvictNormal);
@@ -348,14 +338,6 @@ __global__ void __launch_bounds__(kThreads, 1)
             ++a_seg;
           }
           last_of_m = (tile + 1 >= t_end) || tile_m(tile + 1) != m;
-        }
-        if constexpr (kGemmTimingMode != 0) {   // loads only: hand every stage straight back to the producer
-          for (int ki = 0; ki < k_iters; ++ki, st.next()) {
-            mbar_wait(&full[st.s], st.ph);
-            if (elect_one()) mbar_arrive(&empty[st.s]);
-            __syncwarp();
-          }
-          continue;
         }
         mbar_wait(&t_empty[buf], ((tc >> 1) & 1) ^ 1);
         tc_fence_after();
@@ -400,7 +382,7 @@ __global__ void __launch_bounds__(kThreads, 1)
           tma_load_2d<1>(res_stage + rbuf * kStagingBytes + sl * kBM * 128, &maps.res, &res_full[rbuf], rn0 + sl * 64, rm0,
                          kEvictFirst);
     };
-    if (kTma && has_res && etid == 0 && t_first < t_end && kGemmTimingMode == 0) load_residual(t_first, 0);
+    if (kTma && has_res && etid == 0 && t_first < t_end) load_residual(t_first, 0);
     const bool two_out = p.n_out_bufs == 2;
     const uint32_t sb_addr = smem_u32(sb), out_addr = smem_u32(out_stage), res_addr = smem_u32(res_stage);
     int staged_n0 = -1;
@@ -413,7 +395,7 @@ __global__ void __launch_bounds__(kThreads, 1)
       }
       asm volatile("bar.sync 1, 256;" ::: "memory");
     }
-    for (int tile = t_first; tile < t_end && kGemmTimingMode == 0; tile += t_step, ++tc) {
+    for (int tile = t_first; tile < t_end; tile += t_step, ++tc) {
       const int m0 = tile_m(tile) * kBM;
       const int n0 = tile_n(tile) * BN;
       const uint32_t buf = tc & 1;
@@ -627,7 +609,7 @@ __global__ void __launch_bounds__(kThreads, 1)
 bool wants_a_resident(const GemmParams& p, int BN, bool im2col, size_t max_smem) {
   const int k_iters_h = p.n_terms * p.taps * p.cblocks;
   if (!(!im2col && p.tma_epi && p.n_terms == 1 && p.num_n_tiles >= 2 && (p.res != nullptr || p.num_n_tiles >= 4) &&
-        k_iters_h * kAStage <= 64 * 1024 && p.num_n_tiles * BN <= 4096 && !tuning_flag("DCR_GEMM_NO_ARES")))
+        k_iters_h * kAStage <= 64 * 1024 && p.num_n_tiles * BN <= 4096))
     return false;
   // the resident rows, the all-blocks affine table and the staging tiles must leave at least three W stages; otherwise
   // the layer runs with the default schedule
@@ -736,11 +718,6 @@ int conv_gemm(const ConvGemmDesc& d, cudaStream_t stream) {
     const long long m_tiles = (M + kBM - 1) / kBM;
     while (BN > 64 && ktot >= 1024 && m_tiles * ((d.N + BN - 1) / BN) * 4 <= di->num_sms) BN /= 2;
   }
-  if (d.force_bn) BN = d.force_bn;
-  {
-    const int bn_im2col = tuning_int("DCR_GEMM_BN_IM2COL", 0);   // tuning experiments: tile width of the k x k convolutions
-    if (im2col && (bn_im2col == 64 || bn_im2col == 128 || bn_im2col == 256) && d.N >= bn_im2col) BN = bn_im2col;
-  }
   for (int pl = 0; pl < 3; ++pl) {
     const int pa = std::min(pl, a_planes - 1), pw = std::min(pl, w_planes - 1);
     const __nv_bfloat16* abase = d.in + pa * d.in_plane_stride;
@@ -788,18 +765,14 @@ int conv_gemm(const ConvGemmDesc& d, cudaStream_t stream) {
   p.out_f32 = d.out_f32;
   p.ld_out_f32 = d.ld_out_f32;
   p.act = d.act;
-  p.fast_gelu = (d.n_terms == 1 && p.out_planes <= 1 && !tuning_flag("DCR_GELU_ERF")) ? 1 : 0;
+  p.fast_gelu = (d.n_terms == 1 && p.out_planes <= 1) ? 1 : 0;
   // tile order: with several column blocks and an A matrix larger than what L2 keeps between the passes, m-fastest order
   // streams A from HBM once per column block (ViT-S fc2: 155 MB x 3 = 83 us of HBM time for a 99 us layer)
   const double a_bytes = 2.0 * a_planes * (im2col ? static_cast<double>(d.B) * d.H * d.W * d.C : static_cast<double>(M) * d.C);
   const int order = tuning_int("DCR_GEMM_TILE_ORDER", -1);   // tuning / tests: 0 = m-fastest, 1 = n-fastest, default by size
   p.n_fastest = (order >= 0) ? (order == 1 && p.num_n_tiles >= 2) : (p.num_n_tiles >= 2 && a_bytes > 48e6);
-  if (kGemmTimingMode == 2 && im2col && !windowed) {
-    if (int rc = make_tmap_2d_bf16(&maps.a_flat, d.in, static_cast<uint64_t>(d.B) * d.H * d.W, d.C, d.C, kBM, kBK)) return rc;
-  }
   p.tma_epi = (p.out != nullptr && p.out_planes == 1 && p.out_f32 == nullptr && (p.res == nullptr || p.res_planes == 1) &&
-               (d.act != 2 || p.fast_gelu) &&   // the TMA-store epilogue's compile-time GELU is the tanh form
-               !tuning_flag("DCR_GEMM_DIRECT_EPILOGUE"))
+               (d.act != 2 || p.fast_gelu))   // the TMA-store epilogue's compile-time GELU is the tanh form
                   ? 1
                   : 0;
   if (p.tma_epi) {
@@ -821,7 +794,7 @@ int conv_gemm(const ConvGemmDesc& d, cudaStream_t stream) {
   // ---- CTA-pair form (cta_group::2, 256-row tiles, half a W tile per CTA): plain single-term GEMMs with the TMA-store
   // epilogue whose A rows are not kept resident and that have enough m-tiles to fill the pairs
   const int want_cg2 = tuning_int("DCR_GEMM_CG2", -1);   // 0: never, 1: wherever the kernel form exists, default: policy
-  bool use_cg2 = !im2col && p.tma_epi && p.n_terms == 1 && (BN == 128 || BN == 256) && kGemmTimingMode == 0 && want_cg2 != 0;
+  bool use_cg2 = !im2col && p.tma_epi && p.n_terms == 1 && (BN == 128 || BN == 256) && want_cg2 != 0;
   if (use_cg2 && want_cg2 < 0) {
     // measured per layer at batch 256 (tools/pair_bench.py, B200): 256-wide tiles gain 5-11 % from K = 384 up (ResNet layer3/4
     // reductions 256<-1024, 512<-1024; ViT qkv 1152<-384, ViT-B qkv / fc1); 128-wide residual tiles gain only with many column

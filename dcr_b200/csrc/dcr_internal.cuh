@@ -68,12 +68,11 @@ struct ConvGemmDesc {
   float* out_f32 = nullptr;
   int ld_out_f32 = 0;
   int act = 0;        // 0 none, 1 relu, 2 gelu(erf)
-  int force_bn = 0;   // 0 = auto tile width
   int exact = 0;      // 1 = float64 accumulation on the CUDA cores (conv_exact.cu) instead of the tensor cores
 };
 int conv_gemm(const ConvGemmDesc& d, cudaStream_t stream);
 int conv_exact(const ConvGemmDesc& d, cudaStream_t stream);
-bool conv3x3_halo_eligible(const ConvGemmDesc& d);   // 3x3 / stride 1 / pad 1, fast mode, no residual, W <= 62, N <= 256
+bool conv3x3_halo_eligible(const ConvGemmDesc& d);   // 3x3 / stride 1 / pad 1, fast mode, no residual, W <= 62, N <= 128
 int conv3x3_halo(const ConvGemmDesc& d, cudaStream_t stream);
 // bottleneck_fuse.cu: `a` (1x1 expand + residual + ReLU) followed by `b` (1x1 reduce + ReLU) on a's output, fast mode
 bool expand_reduce_eligible(const ConvGemmDesc& a, const ConvGemmDesc& b, size_t max_smem);

@@ -37,10 +37,11 @@ struct DeviceInfo {
 void count_launch(int n = 1);
 long long launch_count();
 
-// Tuning knobs (DCR_SIM_KP0, DCR_SIM_SETS, DCR_GEMM_NO_ARES, ...) are honoured ONLY when DCR_B200_TUNING=1 is set in the
-// environment: a stray variable cannot change what a benchmark or a test runs.  Every knob selects between variants
-// that produce identical results.  (The timing-experiment modes that produce garbage results are compile-time only:
-// -DDCR_SIM_TIMING_MODE / -DDCR_GEMM_TIMING_MODE / -DDCR_HALO_TIMING_MODE, all 0 in the shipped library.)
+// Tuning switches are honoured ONLY when DCR_B200_TUNING=1 is set in the environment: a stray variable cannot change
+// what a benchmark or a test runs.  Each one selects a variant that gives the same results as the default path, and a
+// GPU test uses each one to compare that variant against the default: DCR_GEMM_CG2, DCR_GEMM_TILE_ORDER and
+// DCR_CONV_NO_HALO (conv_gemm.cu, conv3x3_halo.cu), DCR_POOL_GENERIC (pool_norm.cu), DCR_NO_BLOCK_FUSION
+// (bottleneck_fuse.cu) and DCR_SIM_RESCORE_BLOCK (sim_topk.cu).
 bool tuning_enabled();
 int tuning_int(const char* name, int dflt);
 bool tuning_flag(const char* name);   // true when tuning is enabled and the variable is set (to anything)

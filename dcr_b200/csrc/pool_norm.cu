@@ -810,7 +810,7 @@ int layernorm(const __nv_bfloat16* in, long long in_plane_stride, int planes, in
   p.in_row_stride = in_row_stride; p.gamma = gamma; p.beta = beta; p.eps = eps;
   p.out = out; p.out_plane_stride = out_plane_stride; p.out_f32 = out_f32;
   if (rows == 0) return 0;
-  if (planes == 1 && C % 128 == 0 && C / 128 >= 3 && C / 128 <= 8 && in_row_stride % 8 == 0 && !tuning_flag("DCR_LN_GENERIC")) {
+  if (planes == 1 && C % 128 == 0 && C / 128 >= 3 && C / 128 <= 8 && in_row_stride % 8 == 0) {
     const int blocks = std::min((rows + 15) / 16, di->num_sms * 8);        // 16 half-warps per 256-thread block
     switch (C / 128) {
       case 3: layernorm_fast_kernel<3><<<blocks, 256, 0, stream>>>(p); break;

@@ -40,12 +40,7 @@ constexpr int kWarmTiles = 4;     // tiles replayed at the start of every segmen
 constexpr uint32_t kFull = 0xffffffffu;
 constexpr int kATileBytes = kBlockM * kBlockK * 2;  // 16 KB
 constexpr int kMaxSlotsPerQuery = 512;  // (chunk, unit) segments that may cover one q-tile
-// Timing experiments (results are garbage), compile-time only so that the production issue loops carry no trace of them:
-// 1 = the epilogue loads TMEM but does not scan, 2 = does not even load, 3 = additionally no gallery loads at all.
-#ifndef DCR_SIM_TIMING_MODE
-#define DCR_SIM_TIMING_MODE 0
-#endif
-constexpr int kTimingMode = DCR_SIM_TIMING_MODE;
+constexpr int kCG = 2;            // CTAs per work unit: a CTA pair (cta_group::2)
 
 struct SimParams {
   int nq, ng;
@@ -496,9 +491,8 @@ struct SegWalker {
 };
 
 // ------------------------------------------------------------------------------------------------------------
-// stage 2: the fused kernel.  kCG = 1: one CTA per work unit (UMMA 128x256x16).  kCG = 2: a CTA pair per work
-// unit (UMMA 256x256x16, cta_group::2): each CTA keeps its own 128 queries resident and loads half of every
-// gallery tile, so L2->SMEM traffic per FLOP halves.
+// stage 2: the fused kernel.  A CTA pair per work unit (UMMA 256x256x16, cta_group::2): each CTA keeps its own 128
+// queries resident and loads half of every gallery tile, so L2->SMEM traffic per FLOP is half that of one CTA per unit.
 //
 // Work decomposition: the (q-tile, g-tile) grid is linearised q-major into T = n_qtiles * n_gtiles tiles and cut
 // into gridDim/kCG equal contiguous ranges.  A unit's range is walked as "segments" (maximal runs inside one
@@ -506,7 +500,7 @@ struct SegWalker {
 // replaying the first kWarmTiles tiles.  Segment (unit u, q-tile i) owns candidate slot u + i.
 // kBias: compiled with / without the per-column offset path of query centring.  Both variants are launched; the one
 // that does not match the device-side decision (p.bias_flag) exits at once -- no host synchronisation needed.
-template <int kCG, bool kBias, int kSets>
+template <bool kBias, int kSets>
 __global__ void __launch_bounds__(64 + 128 * kSets, 1)
     sim_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_g,
                     const SimParams p) {
@@ -535,7 +529,7 @@ __global__ void __launch_bounds__(64 + 128 * kSets, 1)
 
   const uint32_t warp = threadIdx.x >> 5;
   const uint32_t lane = threadIdx.x & 31;
-  const uint32_t cta_rank = (kCG == 2) ? cluster_ctarank() : 0;
+  const uint32_t cta_rank = cluster_ctarank();
   const bool leader = (cta_rank == 0);
 
   if (warp == 0 && elect_one()) {
@@ -561,7 +555,7 @@ __global__ void __launch_bounds__(64 + 128 * kSets, 1)
   }
   tc_fence_before();
   __syncthreads();   // CTA-local ordering of the set-up writes (mbarrier init, TMEM slot) for this CTA's own readers ...
-  if constexpr (kCG == 2) cluster_sync();   // ... and the peer CTA's barriers are initialised before any remote arrive
+  cluster_sync();   // ... and the peer CTA's barriers are initialised before any remote arrive
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   if (p.clk && blockIdx.x == 0 && threadIdx.x == 0) {
@@ -600,7 +594,6 @@ __global__ void __launch_bounds__(64 + 128 * kSets, 1)
         for (int j = 0; j < warm + ntiles; ++j) {
           const int gi = g_begin + (j < warm ? j : j - warm);
           const int g_row = gi * kBlockN + static_cast<int>(cta_rank) * kBRows;
-          if constexpr (kTimingMode == 3) continue;   // timing experiment: no gallery loads at all
           for (int kb = 0; kb < p.num_kb; ++kb, st.next()) {
             const uint32_t s = st.s, ph = st.ph;
             mbar_wait(&b_empty[s], ph ^ 1);
@@ -641,7 +634,7 @@ __global__ void __launch_bounds__(64 + 128 * kSets, 1)
           const uint32_t tmem_d = tmem_base + buf * kBlockN;
           for (int kb = 0; kb < p.num_kb; ++kb, st.next()) {
             const uint32_t s = st.s;
-            if constexpr (kTimingMode != 3) mbar_wait(&b_full[s], st.ph);
+            mbar_wait(&b_full[s], st.ph);
             tc_fence_after();
             const uint64_t da = da0 + static_cast<uint64_t>(stream_a ? s * stage_step : static_cast<uint32_t>(kb) * (kATileBytes >> 4));
             const uint64_t db = db0 + static_cast<uint64_t>(s * stage_step);
@@ -649,7 +642,7 @@ __global__ void __launch_bounds__(64 + 128 * kSets, 1)
 #pragma unroll
               for (int k = 0; k < kBlockK / 16; ++k)
                 umma_f16<kCG>(tmem_d, da + 2 * k, db + 2 * k, idesc, (kb | k) != 0);  // +32 B per K=16 step
-              if constexpr (kTimingMode != 3) umma_commit<kCG>(&b_empty[s]);   // frees this B stage (both CTAs) once the MMAs above retire
+              umma_commit<kCG>(&b_empty[s]);   // frees this B stage (both CTAs) once the MMAs above retire
               if (kb == p.num_kb - 1) {
                 umma_commit<kCG>(&t_full[buf]);
                 if (!stream_a && j == warm + ntiles - 1) umma_commit<kCG>(a_empty);
@@ -676,7 +669,7 @@ __global__ void __launch_bounds__(64 + 128 * kSets, 1)
     float* my_carry = carry + set * 4 * kBlockM;
     const int kp = p.kp, cap = p.cap;
     const float* colbias = kBias ? p.col_bias : nullptr;
-    uint32_t tc = 0, dbg = 0;
+    uint32_t tc = 0;
     SegWalker w(p.n_qtiles, p.n_gtiles, p.gchunk, p.n_chunks, unit, n_units);
     while (w.next()) {
       const int qi = w.qi, g_begin = w.g_begin, ntiles = w.ntiles;
@@ -725,15 +718,8 @@ __global__ void __launch_bounds__(64 + 128 * kSets, 1)
         auto release = [&]() {   // this warp's columns of the accumulator buffer are in registers
           tc_fence_before();
           __syncwarp();
-          if (lane == 0) {
-            if constexpr (kCG == 2) mbar_arrive_cluster(&t_empty[buf], 0);
-            else mbar_arrive(&t_empty[buf]);
-          }
+          if (lane == 0) mbar_arrive_cluster(&t_empty[buf], 0);
         };
-        if constexpr (kTimingMode >= 2) {   // timing experiment: do not even read the accumulator (results are meaningless)
-          release();
-          return;
-        }
         // TMEM read pipeline: chunk i+1 is in flight while chunk i is scanned
         tmem_ld_32x32(taddr, ra);
 #pragma unroll 1
@@ -741,22 +727,14 @@ __global__ void __launch_bounds__(64 + 128 * kSets, 1)
           tmem_ld_wait_dep(ra);
           tmem_ld_32x32(taddr + (ch + 1) * 32, rb);
           if (tail) mask_tail(ra, gcol0 + ch * 32, p.ng);
-          if constexpr (kTimingMode == 0) {
-            if constexpr (kWarm) warm_chunk<false>(ra, sb ? sb + ch * 32 : nullptr, gcol0 + ch * 32, p.ng, slot);
-            else scan_chunk<false>(ra, sb ? sb + ch * 32 : nullptr, gcol0 + ch * 32, p.ng, thr, cnt, my_list, warp_list, kp, cap, lane);
-          } else {
-            dbg ^= ra[0] ^ ra[31];
-          }
+          if constexpr (kWarm) warm_chunk<false>(ra, sb ? sb + ch * 32 : nullptr, gcol0 + ch * 32, p.ng, slot);
+          else scan_chunk<false>(ra, sb ? sb + ch * 32 : nullptr, gcol0 + ch * 32, p.ng, thr, cnt, my_list, warp_list, kp, cap, lane);
           tmem_ld_wait_dep(rb);
           if (ch + 2 < kSetCols / 32) tmem_ld_32x32(taddr + (ch + 2) * 32, ra);
           else release();
           if (tail) mask_tail(rb, gcol0 + (ch + 1) * 32, p.ng);
-          if constexpr (kTimingMode == 0) {
-            if constexpr (kWarm) warm_chunk<false>(rb, sb ? sb + (ch + 1) * 32 : nullptr, gcol0 + (ch + 1) * 32, p.ng, slot);
-            else scan_chunk<false>(rb, sb ? sb + (ch + 1) * 32 : nullptr, gcol0 + (ch + 1) * 32, p.ng, thr, cnt, my_list, warp_list, kp, cap, lane);
-          } else {
-            dbg ^= rb[0] ^ rb[31];
-          }
+          if constexpr (kWarm) warm_chunk<false>(rb, sb ? sb + (ch + 1) * 32 : nullptr, gcol0 + (ch + 1) * 32, p.ng, slot);
+          else scan_chunk<false>(rb, sb ? sb + (ch + 1) * 32 : nullptr, gcol0 + (ch + 1) * 32, p.ng, thr, cnt, my_list, warp_list, kp, cap, lane);
         }
       };
       if (warm > 0) {
@@ -787,14 +765,14 @@ __global__ void __launch_bounds__(64 + 128 * kSets, 1)
         if (static_cast<int>(lane) < n) p.cand[(slot_row0 + L) * kKPMax + lane] = warp_list[L + lane * 128];
       }
       p.cand_cnt[slot_row0 + lane] = cnt;
-      p.cand_thr[slot_row0 + lane] = (kTimingMode != 0 && dbg == 0x12345678u) ? 0.f : thr;   // keeps `dbg` live in the timing modes
+      p.cand_thr[slot_row0 + lane] = thr;
       __syncwarp();
     }
   }
 
   // teardown
   tc_fence_before();
-  if constexpr (kCG == 2) cluster_sync(); else __syncthreads();
+  cluster_sync();
   if (warp == 2) tmem_dealloc<kCG>(tmem_base, 512);
   if (p.clk && blockIdx.x == 0 && threadIdx.x == 0) {
     p.clk[2] = clock64();
@@ -1525,7 +1503,6 @@ __global__ void __launch_bounds__(256)
 }
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
-int env_int(const char* name, int dflt);
 
 // launch geometry of one fused pass over nq queries
 struct PassPlan {
@@ -1536,7 +1513,7 @@ struct PassPlan {
 };
 
 struct SimPlan {
-  int cg, d_pad, num_kb, ng_pad, n_gtiles, rows_per_qtile;
+  int d_pad, num_kb, ng_pad, n_gtiles, rows_per_qtile;
   int stream_a;  // d_pad > 512: query tile streamed with the gallery k-blocks
   int max_sets;  // upper bound for PassPlan::n_sets (1 or 2)
   int gchunk, n_chunks;   // preferred gallery chunking (a pass may use fewer chunks)
@@ -1555,7 +1532,7 @@ int plan_pass(int nq, int kp, const SimPlan& sp, int num_sms, size_t max_smem, i
   pp->kp = kp;
   // ---- shared memory: resident A + stages*B + n_sets * cap KB of lists + barriers + carried thresholds ----
   const size_t a_bytes = sp.stream_a ? 0 : static_cast<size_t>(sp.num_kb) * kATileBytes;
-  const size_t b_tile = static_cast<size_t>(kBlockN / sp.cg) * kBlockK * 2 + (sp.stream_a ? kATileBytes : 0);
+  const size_t b_tile = static_cast<size_t>(kBlockN / kCG) * kBlockK * 2 + (sp.stream_a ? kATileBytes : 0);
   const size_t fixed = 1024 /*align slack*/ + 256 /*barriers*/ + 4096 /*carried thresholds*/;
   auto fits = [&](int st, int cp, int sets) {
     return max_smem >= a_bytes + st * b_tile + static_cast<size_t>(cp) * 1024 * sets + fixed;
@@ -1563,15 +1540,11 @@ int plan_pass(int nq, int kp, const SimPlan& sp, int num_sms, size_t max_smem, i
   // two epilogue warp sets whenever their lists (at least kp + 8 entries per row and set) fit next to 3 B stages
   int sets = (sp.max_sets >= 2 && fits(3, kp + 8, 2)) ? 2 : 1;
   int cap = kp + (sets == 2 ? 8 : 16);
-  const int cap_max = std::max(cap, std::min(64, env_int("DCR_SIM_CAP", 64)));
   int stages = 2;
-  DCR_REQUIRE(fits(stages, cap, sets), "sim_topk: not enough shared memory (%zu B) for d=%d k=%d cta_group=%d", max_smem,
-              d, k, sp.cg);
+  DCR_REQUIRE(fits(stages, cap, sets), "sim_topk: not enough shared memory (%zu B) for d=%d k=%d", max_smem, d, k);
   // priorities: 3 B stages, then list capacity up to 64 (fewer compactions), then more stages (up to 8)
   if (fits(3, cap, sets)) stages = 3;
-  const int want_stages = env_int("DCR_SIM_STAGES", 0);
-  if (want_stages > 3 && fits(want_stages, cap, sets)) stages = want_stages;
-  while (cap < cap_max && fits(stages, cap + 1, sets)) ++cap;
+  while (cap < 64 && fits(stages, cap + 1, sets)) ++cap;
   while (stages < 8 && fits(stages + 1, cap, sets)) ++stages;
   pp->cap = cap;
   pp->stages = stages;
@@ -1585,7 +1558,7 @@ int plan_pass(int nq, int kp, const SimPlan& sp, int num_sms, size_t max_smem, i
   long long span_total = 0;
   for (;;) {
     const long long T = static_cast<long long>(pp->n_qtiles) * pp->gchunk;   // tiles of one (full) gallery chunk
-    units = num_sms / sp.cg;
+    units = num_sms / kCG;
     if (T < units) units = static_cast<int>(std::max<long long>(1, T));
     // per chunk a q-tile is covered by at most ceil(tiles_in_chunk / (T_c / units)) + 1 units
     span_total = 0;
@@ -1612,28 +1585,23 @@ int plan_pass(int nq, int kp, const SimPlan& sp, int num_sms, size_t max_smem, i
   return 0;
 }
 
-int env_int(const char* name, int dflt) { return tuning_int(name, dflt); }   // honoured only under DCR_B200_TUNING=1
-
-int make_plan(int nq, int ng, int d, int k, int cg, int num_sms, size_t max_smem, SimPlan* pl) {
+int make_plan(int nq, int ng, int d, int k, int num_sms, size_t max_smem, SimPlan* pl) {
   DCR_REQUIRE(nq >= 1 && ng >= 1 && d >= 1, "sim_topk: empty problem (nq=%d ng=%d d=%d)", nq, ng, d);
   DCR_REQUIRE(d <= kMaxDim, "sim_topk: descriptor dim %d > %d not supported", d, kMaxDim);
   DCR_REQUIRE(k >= 1 && k <= 16, "sim_topk: k=%d outside [1,16]", k);
   DCR_REQUIRE(k <= ng, "sim_topk: k=%d > gallery size %d", k, ng);
-  DCR_REQUIRE(cg == 1 || cg == 2, "sim_topk: cta group must be 1 or 2");
-  pl->cg = cg;
   pl->d_pad = static_cast<int>(align_up(d, kBlockK));
   pl->num_kb = pl->d_pad / kBlockK;
   pl->stream_a = pl->num_kb > kMaxKB ? 1 : 0;
-  pl->rows_per_qtile = kBlockM * cg;
+  pl->rows_per_qtile = kBlockM * kCG;
   // Two epilogue warp sets (two warps per TMEM lane quadrant, each with its own lists for one column half) pay off when
   // few candidates are kept: measured on B200 (10k x 100k x 512) k = 1: 0.79 ms vs 0.82 ms and no second-chance pass
   // (each segment keeps 2 x 4 candidates); k = 10: slower (the lists of two sets only fit with a small capacity).
-  // DCR_SIM_SETS=1|2 overrides.
-  pl->max_sets = (cg == 2) ? std::max(1, std::min(2, env_int("DCR_SIM_SETS", k <= 2 ? 2 : 1))) : 1;
+  pl->max_sets = k <= 2 ? 2 : 1;
   pl->n_gtiles = (ng + kBlockN - 1) / kBlockN;
   pl->ng_pad = pl->n_gtiles * kBlockN;
-  // gallery chunks of ~DCR_SIM_CHUNK_MB of bf16 rows: the units sweep one chunk at a time so that it stays L2 resident
-  const long long chunk_bytes = static_cast<long long>(env_int("DCR_SIM_CHUNK_MB", 40)) << 20;
+  // gallery chunks of ~40 MB of bf16 rows: the units sweep one chunk at a time so that it stays L2 resident
+  const long long chunk_bytes = 40ll << 20;
   int gchunk = static_cast<int>(std::max<long long>(16, chunk_bytes / (static_cast<long long>(kBlockN) * pl->d_pad * 2)));
   int n_chunks = (pl->n_gtiles + gchunk - 1) / gchunk;
   if (n_chunks > 64) n_chunks = 64;
@@ -1645,9 +1613,7 @@ int make_plan(int nq, int ng, int d, int k, int cg, int num_sms, size_t max_smem
   // bound of the k-th score; such queries get a second chance with 32 candidates before the brute-force path
   // k in 6..10 keeps 12 (measured on B200, 10k x 100k x 512, k = 10: 1.20 ms with 16, 1.14 ms with 12, 1.10 ms with 10;
   // two spare candidates per segment keep the second-chance pass rare)
-  int kp0 = (k <= 2) ? 4 : (k <= 5 ? 8 : (k <= 10 ? 12 : 32));
-  kp0 = env_int("DCR_SIM_KP0", kp0);
-  DCR_REQUIRE(kp0 >= 1 && kp0 <= kKPMax, "sim_topk: DCR_SIM_KP0 must be in [1, 32]");
+  const int kp0 = (k <= 2) ? 4 : (k <= 5 ? 8 : (k <= 10 ? 12 : 32));
   DCR_REQUIRE(kp0 >= k, "sim_topk: first-pass candidate count %d < k=%d", kp0, k);
   pl->kp0 = kp0;
   pl->kp1 = (kp0 < kKPMax) ? kKPMax : 0;
@@ -1688,11 +1654,6 @@ int make_plan(int nq, int ng, int d, int k, int cg, int num_sms, size_t max_smem
   return 0;
 }
 
-int default_cg() {
-  const int cg = tuning_int("DCR_SIM_CTA_GROUP", 2);
-  return (cg == 1 || cg == 2) ? cg : 2;
-}
-
 struct PassBuffers {
   uint2* cand;
   int* ccnt;
@@ -1705,7 +1666,7 @@ int launch_fused(const SimPlan& pl, const PassPlan& pp, const __nv_bfloat16* qb,
                  unsigned long long* clk, unsigned int* gthr, cudaStream_t stream) {
   CUtensorMap tq, tg;
   if (int rc = make_tmap_2d_bf16(&tq, qb, pp.nq_pad, pl.d_pad, pl.d_pad, kBlockM, kBlockK)) return rc;
-  if (int rc = make_tmap_2d_bf16(&tg, gb, pl.ng_pad, pl.d_pad, pl.d_pad, kBlockN / pl.cg, kBlockK)) return rc;
+  if (int rc = make_tmap_2d_bf16(&tg, gb, pl.ng_pad, pl.d_pad, pl.d_pad, kBlockN / kCG, kBlockK)) return rc;
   SimParams p;
   p.nq = pp.nq;
   p.ng = ng;
@@ -1726,15 +1687,15 @@ int launch_fused(const SimPlan& pl, const PassPlan& pp, const __nv_bfloat16* qb,
   p.thr_init = thr_init;
   p.clk = clk;
   p.gthr = gthr;
-  if (gthr) DCR_CUDA_CHECK(cudaMemsetAsync(gthr, 0, static_cast<size_t>(pp.nq_pad) * 4, stream));
+  DCR_CUDA_CHECK(cudaMemsetAsync(gthr, 0, static_cast<size_t>(pp.nq_pad) * 4, stream));
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(pp.n_units * pl.cg);
+  cfg.gridDim = dim3(pp.n_units * kCG);
   cfg.blockDim = dim3(64 + 128 * pp.n_sets);
   cfg.dynamicSmemBytes = pp.smem_bytes;
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = pl.cg;
+  attr[0].val.clusterDim.x = kCG;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
@@ -1745,19 +1706,13 @@ int launch_fused(const SimPlan& pl, const PassPlan& pp, const __nv_bfloat16* qb,
     count_launch();
     return 0;
   };
-  // the variant without the offset path always runs unless the device flag says otherwise; the offset variant is only
-  // launched when query centring is possible at all (it returns immediately when the flag is 0)
-  if (pl.cg == 2 && pp.n_sets == 2) {
-    if (int rc = launch(sim_topk_kernel<2, false, 2>)) return rc;
-    if (col_bias) return launch(sim_topk_kernel<2, true, 2>);
-  } else if (pl.cg == 2) {
-    if (int rc = launch(sim_topk_kernel<2, false, 1>)) return rc;
-    if (col_bias) return launch(sim_topk_kernel<2, true, 1>);
-  } else {
-    if (int rc = launch(sim_topk_kernel<1, false, 1>)) return rc;
-    if (col_bias) return launch(sim_topk_kernel<1, true, 1>);
+  // both variants are launched; the one that does not match the device flag of query centring returns at once
+  if (pp.n_sets == 2) {
+    if (int rc = launch(sim_topk_kernel<false, 2>)) return rc;
+    return launch(sim_topk_kernel<true, 2>);
   }
-  return 0;
+  if (int rc = launch(sim_topk_kernel<false, 1>)) return rc;
+  return launch(sim_topk_kernel<true, 1>);
 }
 
 }  // namespace
@@ -1780,7 +1735,7 @@ int split_rescore(const float* q, const float* g, int nq, int d, int n_chunks, i
 size_t sim_topk_workspace_size(int nq, int ng, int d, int k) {
   const DeviceInfo* di = device_info();
   SimPlan pl;
-  if (make_plan(nq, ng, d, k, default_cg(), di ? di->num_sms : 148, di ? di->max_smem_optin : 232448, &pl) != 0)
+  if (make_plan(nq, ng, d, k, di ? di->num_sms : 148, di ? di->max_smem_optin : 232448, &pl) != 0)
     return 0;
   return pl.total;
 }
@@ -1791,9 +1746,8 @@ int sim_topk(const float* q, int nq, const float* g, int ng, int d, int k, long 
   const DeviceInfo* di = device_info();
   if (!di) return -2;
   DCR_REQUIRE(di->cc_major == 10, "sim_topk: this build targets sm_100a; device reports sm_%d%d", di->cc_major, di->cc_minor);
-  const int cg = default_cg();
   SimPlan pl;
-  if (int rc = make_plan(nq, ng, d, k, cg, di->num_sms, di->max_smem_optin, &pl)) return rc;
+  if (int rc = make_plan(nq, ng, d, k, di->num_sms, di->max_smem_optin, &pl)) return rc;
   DCR_REQUIRE(ws != nullptr && ws_bytes >= pl.total, "sim_topk: workspace too small (%zu < %zu)", ws_bytes, pl.total);
   DCR_REQUIRE((reinterpret_cast<uintptr_t>(ws) & 255) == 0, "sim_topk: workspace must be 256-byte aligned");
   DCR_REQUIRE((reinterpret_cast<uintptr_t>(q) & 15) == 0 && (reinterpret_cast<uintptr_t>(g) & 15) == 0 && d % 4 == 0,
@@ -1820,9 +1774,8 @@ int sim_topk(const float* q, int nq, const float* g, int ng, int d, int k, long 
   auto* counts = reinterpret_cast<int*>(w + pl.off_counts);   // [0] flagged by pass 0, [1] flagged by pass 1
   auto* exact = reinterpret_cast<double*>(w + pl.off_exact);
   auto* clk = reinterpret_cast<unsigned long long*>(w + pl.off_clk);
-  unsigned int* gthr = env_int("DCR_SIM_SHARE_THR", 1) ? reinterpret_cast<unsigned int*>(w + pl.off_gthr) : nullptr;
+  auto* gthr = reinterpret_cast<unsigned int*>(w + pl.off_gthr);
 
-  const bool centre = env_int("DCR_SIM_CENTER", 1) != 0;
   DCR_CUDA_CHECK(cudaMemsetAsync(gmax, 0, 16, stream));
   DCR_CUDA_CHECK(cudaMemsetAsync(counts, 0, 16, stream));   // [0],[1] flagged counts, [2] query-centring flag
   const int conv_blocks = di->num_sms * 8;
@@ -1843,22 +1796,19 @@ int sim_topk(const float* q, int nq, const float* g, int ng, int d, int k, long 
     }
     return 0;
   };
-  if (centre) {
-    if (int rc = sampled_mean(g, ng, mu, false)) return rc;    // gallery centre mu (always used)
-    if (int rc = sampled_mean(q, nq, nu, true)) return rc;     // query centre nu + the decision whether to use it
-  }
+  if (int rc = sampled_mean(g, ng, mu, false)) return rc;    // gallery centre mu (always used)
+  if (int rc = sampled_mean(q, nq, nu, true)) return rc;     // query centre nu + the decision whether to use it
   // q' = q - nu, g' = g - mu:  q.g = q'.g' + nu.g' + q.mu  -- the tensor cores see only the centred parts, nu.g' is a
   // per-gallery-row offset added to the accumulator columns, q.mu a per-query constant that cannot change the ranking
   // d_pad <= 256: 2 loads per lane cover the row; otherwise 4 per round (512 dims = one round)
   auto convert = (pl.d_pad <= 256) ? to_bf16_rows_kernel<2> : to_bf16_rows_kernel<4>;
-  convert<<<conv_blocks, 256, 0, stream>>>(q, nq, d, pl.p0.nq_pad, pl.d_pad, centre ? nu : nullptr, qb, qnh, qnr, qnx, nullptr,
+  convert<<<conv_blocks, 256, 0, stream>>>(q, nq, d, pl.p0.nq_pad, pl.d_pad, nu, qb, qnh, qnr, qnx, nullptr,
                                            nullptr, nullptr, qflag, nullptr);
   count_launch();
-  convert<<<conv_blocks, 256, 0, stream>>>(g, ng, d, pl.ng_pad, pl.d_pad, centre ? mu : nullptr, gb, nullptr, nullptr, nullptr,
-                                           gmax, centre ? nu : nullptr, centre ? bias : nullptr, nullptr, qflag);
+  convert<<<conv_blocks, 256, 0, stream>>>(g, ng, d, pl.ng_pad, pl.d_pad, mu, gb, nullptr, nullptr, nullptr,
+                                           gmax, nu, bias, nullptr, qflag);
   count_launch();
   DCR_CUDA_CHECK(cudaGetLastError());
-  const float* col_bias = centre ? bias : nullptr;
 
   // CUDA events around the first fused pass only (thread-local, created once): bench.py's roofline numerator
   // (events belong to the device that was current when they were created: one pair per device)
@@ -1870,7 +1820,7 @@ int sim_topk(const float* q, int nq, const float* g, int ng, int d, int k, long 
     DCR_CUDA_CHECK(cudaEventCreate(&ev1));
   }
   DCR_CUDA_CHECK(cudaEventRecord(ev0, stream));
-  if (int rc = launch_fused(pl, pl.p0, qb, gb, ng, pb, col_bias, qflag, nullptr, clk, gthr, stream)) return rc;
+  if (int rc = launch_fused(pl, pl.p0, qb, gb, ng, pb, bias, qflag, nullptr, clk, gthr, stream)) return rc;
   DCR_CUDA_CHECK(cudaEventRecord(ev1, stream));
 
   auto rescore = [&](const PassPlan& pp, const int* qmap, int* flagged, int* n_flagged, float* thr_next) -> int {
@@ -1883,7 +1833,7 @@ int sim_topk(const float* q, int nq, const float* g, int ng, int d, int k, long 
       DCR_CUDA_CHECK(cudaFuncSetAttribute(rescore_select_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
       rescore_select_warp_kernel<<<(pp.nq + kRescoreWarps - 1) / kRescoreWarps, 32 * kRescoreWarps, smem, stream>>>(
           q, g, pp.nq, d, k, pp.n_qtiles, pl.n_gtiles, pp.gchunk, pp.n_chunks, pp.n_units, pl.rows_per_qtile, pp.n_sets, pl.d_pad,
-          pb.cand, pb.ccnt, pb.cthr, qmap, centre ? mu : nullptr, centre ? nu : nullptr, qflag, qnh, qnr, qnx, gmax, g_index_base,
+          pb.cand, pb.ccnt, pb.cthr, qmap, mu, nu, qflag, qnh, qnr, qnx, gmax, g_index_base,
           g_index_stride, out_scores, out_idx, flagged, n_flagged, thr_next, pp.max_cand);
       count_launch();
       DCR_CUDA_CHECK(cudaGetLastError());
@@ -1895,7 +1845,7 @@ int sim_topk(const float* q, int nq, const float* g, int ng, int d, int k, long 
     rescore_select_kernel<<<pp.nq, 128, rs_smem, stream>>>(
         q, g, nq, ng, d, k, pp.n_qtiles, pl.n_gtiles, pp.gchunk, pp.n_chunks, pp.n_units, pl.rows_per_qtile, pp.n_sets, pl.d_pad,
         pb.cand, pb.ccnt,
-        pb.cthr, qmap, centre ? mu : nullptr, centre ? nu : nullptr, qflag, qnh, qnr, qnx, gmax, g_index_base, g_index_stride, out_scores, out_idx,
+        pb.cthr, qmap, mu, nu, qflag, qnh, qnr, qnx, gmax, g_index_base, g_index_stride, out_scores, out_idx,
         flagged, n_flagged, thr_next, pp.max_cand);
     count_launch();
     DCR_CUDA_CHECK(cudaGetLastError());
@@ -1919,7 +1869,7 @@ int sim_topk(const float* q, int nq, const float* g, int ng, int d, int k, long 
     gather_rows_kernel<<<std::min(di->num_sms * 8, (p1.nq_pad * (pl.d_pad / 8) + 255) / 256), 256, 0, stream>>>(
         qb, flag0, n_second, p1.nq_pad, pl.d_pad, qb1);
     count_launch();
-    if (int rc = launch_fused(pl, p1, qb1, gb, ng, pb, col_bias, qflag, thr1, nullptr, gthr, stream)) return rc;
+    if (int rc = launch_fused(pl, p1, qb1, gb, ng, pb, bias, qflag, thr1, nullptr, gthr, stream)) return rc;
     if (int rc = rescore(p1, flag0, flag1, counts + 1, nullptr)) return rc;
     DCR_CUDA_CHECK(cudaMemcpyAsync(h_counts, counts, 8, cudaMemcpyDeviceToHost, stream));
     DCR_CUDA_CHECK(cudaStreamSynchronize(stream));
@@ -1954,8 +1904,8 @@ int sim_topk(const float* q, int nq, const float* g, int ng, int d, int k, long 
                                                                static_cast<double>(h_clk[3] - h_clk[1]))
                                           : 0.f;
     stats->n_sets = pl.p0.n_sets;
-    stats->cta_group = cg;
-    stats->grid = pl.p0.n_units * cg;
+    stats->cta_group = kCG;
+    stats->grid = pl.p0.n_units * kCG;
     stats->smem_bytes = static_cast<int>(pl.p0.smem_bytes);
     stats->stages = pl.p0.stages;
     stats->kp = pl.p0.kp;
